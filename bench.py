@@ -8,6 +8,8 @@ composite + MSE against the target images, and back-propagate to every leaf para
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--workload dtu|bmvs|stress]     our arm (torchrun launches N ranks)
   python bench.py --impl reference ...                            the reference's algorithm on the host cores (oracle port)
+  python bench.py ... --dump-outputs DIR       also write what the last timed step computed (losses, every leaf gradient)
+                                               as DIR/<name>.npy, to compare two builds output for output
 
 Workloads = BASELINE.json configs: dtu = configs[1]/[2] (the metric's configuration and the default), bmvs = configs[3],
 stress = configs[4].  N > 1 is STRONG scaling: the step's views are split over the ranks at (view, 16-row band) granularity.
@@ -36,6 +38,7 @@ WORKLOADS = {
                                            '800x800, K=25, 128^2 block textures, 256^2 env textures'),
 }
 SEED = 227391          # configs/dtu/default.yml:42
+DUMP_LIMIT = 64 << 20  # bytes --dump-outputs may write
 PASS_BYTES = 30e9      # views of a step are processed in passes of at most this much workspace (gradients accumulate)
 
 
@@ -133,6 +136,21 @@ def synthetic_inputs(w):
     return {'imgs': imgs, 'R': R, 'T': T, 'K': K[None].expand(B, -1, -1).contiguous()}
 
 
+def dump_outputs(out_dir, model, losses, loss_suffix=''):
+    """the step's result as its caller holds it: the loss terms and the gradient of every leaf parameter (p.grad), float32"""
+    import numpy as np
+    arrays = {f'loss_{k}{loss_suffix}': v.detach().float().reshape(1) for k, v in losses.items()}
+    for n, p in model.named_parameters():
+        if p.requires_grad:
+            arrays[f'grad_{n}'] = (p.grad if p.grad is not None else torch.zeros_like(p)).detach().float()
+    total = sum(v.numel() * 4 for v in arrays.values())
+    if total > DUMP_LIMIT:
+        raise RuntimeError(f'--dump-outputs: {total} bytes exceed the {DUMP_LIMIT} byte limit')
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in arrays.items():
+        np.save(os.path.join(out_dir, f'{k}.npy'), v.cpu().numpy())
+
+
 def make_passes(local, rows, w):
     """split this rank's views into passes of equal shape: [{imgs, R, T, K, rows}] (host, pinned).  Padding entries of the
     last pass repeat view 0 with an EMPTY row range, so that one captured graph serves every pass."""
@@ -197,13 +215,14 @@ def run_ours(args):
 
     def step_eager(collective=True):
         for i, p in enumerate(dev_passes):
-            vp.forward_backward(p, None, already_sharded=True, n_total_views=B, all_reduce=collective and inside)
+            losses = vp.forward_backward(p, None, already_sharded=True, n_total_views=B, all_reduce=collective and inside)
             if acc is not None:
                 acc.copy_(vp.bucket.flat) if i == 0 else acc.add_(vp.bucket.flat)
         if acc is not None:
             vp.bucket.flat.copy_(acc)
         if collective and not inside:
             vp.bucket.all_reduce(vp.group)
+        return losses
 
     graphed = piped = None
     nocoll = None
@@ -220,13 +239,14 @@ def run_ours(args):
             return step_eager(collective)
         g = graphed if collective else nocoll
         for i, p in enumerate(dev_passes):
-            g.run(p if n_pass > 1 else None, all_reduce=False)          # a collective captured in the graph runs regardless
+            losses = g.run(p if n_pass > 1 else None, all_reduce=False)      # a collective captured in the graph runs regardless
             if acc is not None:
                 acc.copy_(vp.bucket.flat) if i == 0 else acc.add_(vp.bucket.flat)
         if acc is not None:
             vp.bucket.flat.copy_(acc)
         if collective and not g.capture_all_reduce and not inside:
             vp.bucket.all_reduce(vp.group)
+        return losses
 
     def step_e2e():
         """the public API with HOST buffers: every pass's inputs are copied H2D from pinned memory (the next pass's while
@@ -256,6 +276,8 @@ def run_ours(args):
             dist.barrier()
         torch.cuda.synchronize()
 
+    last = {}
+
     def timed(fn, steps):
         evs = []
         barrier()
@@ -263,7 +285,7 @@ def run_ours(args):
             flush.zero_()
             a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
             a.record()
-            fn()
+            last['losses'] = fn()
             b.record()
             evs.append((a, b))
         barrier()
@@ -282,8 +304,13 @@ def run_ours(args):
     sampler = ClockSampler(local) if rank == 0 else None
     if sampler:
         sampler.start()
-    ms_local = timed(step_resident, args.steps)
-    clocks = sampler.summary() if sampler else None
+    try:
+        ms_local = timed(step_resident, args.steps)
+    finally:
+        clocks = sampler.summary() if sampler else None          # stops the sampling process
+    if args.dump_outputs and rank == 0:
+        # a step of several passes keeps only its last pass's loss terms (its gradients are the sum over the passes)
+        dump_outputs(args.dump_outputs, model, last['losses'], '' if n_pass == 1 else '_last_pass')
     # the same steps without the gradient collective: what the all-reduce adds to a step when it is exposed
     ms_nocoll_local = timed(lambda: step_resident(False), args.steps) if world > 1 else ms_local
 
@@ -446,7 +473,8 @@ def run_reference(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument('--gpus', type=int, default=1)
-    ap.add_argument('--steps', type=int, default=100)
+    ap.add_argument('--steps', type=int, default=None,
+                    help='timed steps (default: 100 on dtu, 10 on the larger workloads, 5 with --impl reference)')
     ap.add_argument('--warmup', type=int, default=5)
     ap.add_argument('--impl', default='ours', choices=['ours', 'reference'])
     ap.add_argument('--workload', default='dtu', choices=sorted(WORKLOADS))
@@ -457,12 +485,18 @@ def main():
                          'step is split over 4 or more GPUs (short launches whose tails then overlap)')
     ap.add_argument('--no-cpu-baseline', action='store_true')
     ap.add_argument('--no-graph', action='store_true', help='submit the step eagerly instead of replaying a CUDA graph')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help="write the last timed step's loss terms and leaf gradients as DIR/<name>.npy (float32)")
     args = ap.parse_args()
-    if args.workload != 'dtu' and args.steps == 100:
-        args.steps = 10              # the larger workloads take 10-100x longer per step: keep the default run within minutes
+    if args.steps is None:
+        # the larger workloads take 10-100x longer per step, and a reference step is a bounded CPU sample: keep the
+        # default run within minutes
+        args.steps = 5 if args.impl == 'reference' else 100 if args.workload == 'dtu' else 10
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
     if args.impl == 'reference':
-        if args.steps > 5:
-            args.steps = 5          # each step is a bounded CPU sample; keep the whole run within minutes
+        if args.dump_outputs:
+            ap.error('--dump-outputs applies to our arm')
         run_reference(args)
     else:
         run_ours(args)

@@ -1,18 +1,19 @@
-"""AST-extraction of the reference's own pure-torch functions (only possible where /root/reference exists).
+"""AST-extraction of the reference's own pure-torch functions from a checkout of the original project (used by
+tests/golden/make_golden.py to generate the golden vectors; the tests themselves read only tests/golden/).
 
-Nothing is copied into the repo: the function source is read from the reference checkout at test time, compiled
-in a scratch namespace and called, so the comparison is against the reference's code itself."""
+Nothing is copied into the repo: the function source is read from the reference checkout, compiled in a scratch
+namespace and called, so the vectors are produced by the reference's code itself."""
 import ast
 import os
 
 import numpy as np
 import torch
 
-REF = '/root/reference'
+REF = None          # path of the reference checkout; set by the caller (make_golden.py --reference DIR)
 
 
 def have_reference():
-    return os.path.isdir(os.path.join(REF, 'src'))
+    return REF is not None and os.path.isdir(os.path.join(REF, 'src'))
 
 
 def extract(relpath, names, extra_ns=None):

@@ -1,14 +1,16 @@
 """Drives the reference's UNMODIFIED `src/trainer.py` (+ optimizer.py, scheduler.py, utils/*, configs/dtu/*.yml) on this repo's
-model -- run as a subprocess by tests/test_reference_trainer.py, only where the reference checkout exists.
+model, from a checkout of the reference (monniert/differentiable-blocksworld):
 
-    python tests/ref_trainer_driver.py <run_dir> [--iters N]
+    python tests/ref_trainer_driver.py --reference <checkout> <run_dir> [--iters N]
+
+It prints one `DRIVER_RESULT <json>` line: loss names, Adam groups, moved parameters, checkpoint keys, metrics rows, resume.
 
 What is swapped (INTEGRATION.md A, nothing in the reference tree is edited or copied):
   * `model.create_model`                 -> dbw_b200.dbw.create_model   (the drop-in)
   * `dataset.create_train_val_test_loader` -> a synthetic multi-view loader (no DTU images on disk here)
   * missing third-party modules          -> dbw_b200.compat stand-ins
 
-With a GPU the model renders for real.  WITHOUT one (the authoring container) the product renderer refuses to run -- there is
+With a GPU the model renders for real.  WITHOUT one the product renderer refuses to run -- there is
 no CPU fallback, by design -- so this driver replaces the model's three render entry points by parameter-touching dummies and
 says so: what the run then proves is the whole trainer <-> model surface (config parsing, loss names, Adam groups,
 schedules, metrics, visualisation calls, checkpoints, resume), not pixels."""
@@ -19,7 +21,6 @@ import sys
 from pathlib import Path
 
 REPO = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = '/root/reference'
 sys.path.insert(0, REPO)
 
 import torch  # noqa: E402
@@ -76,8 +77,10 @@ def stub_render_entry_points():
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument('run_dir')
+    ap.add_argument('--reference', required=True, help='checkout of the reference')
     ap.add_argument('--iters', type=int, default=3)
     args = ap.parse_args()
+    REF = os.path.realpath(args.reference)
     shimmed = compat.install()
     sys.path.insert(0, os.path.join(REF, 'src'))
     import dataset as ref_dataset

@@ -1,14 +1,12 @@
-"""CPU: the oracle against the committed golden vectors (tests/golden/, generator make_golden.py) and -- where the
-reference checkout is present -- against the reference's own functions extracted with `ast`."""
+"""CPU: the oracle against the committed golden vectors (tests/golden/, generator make_golden.py), among them the outputs
+of the reference's own functions (extracted with `ast` from a reference checkout when the vectors were generated)."""
 import os
-from types import SimpleNamespace
 
 import numpy as np
 import pytest
 import torch
 
 from oracle import dbw_path as D, pt3d
-from tests._refextract import extract, extract_method, have_reference
 
 GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), 'golden')
 
@@ -52,12 +50,12 @@ def test_cube_primitive_matches_reference_golden():
     assert torch.equal(ov.reshape(-1, 3), g['plane_verts']) and torch.equal(of.reshape(-1, 3), g['plane_faces'])
 
 
-@pytest.mark.skipif(not have_reference(), reason='needs the reference checkout (/root/reference)')
 def test_obj_loader_reads_the_reference_primitives():
+    """the reference's primitives/*.obj, stored verbatim under tests/golden/primitives/"""
     import dbw_b200  # noqa: F401
     from dbw_b200 import geometry as G
     for name, (v, f) in (('cube', G.unit_cube()), ('plane', G.unit_plane())):
-        lv, lf = G.load_obj(f'/root/reference/primitives/{name}.obj')
+        lv, lf = G.load_obj(os.path.join(GOLD, 'primitives', f'{name}.obj'))
         assert torch.equal(lv, v) and torch.equal(lf, f), name
 
 
@@ -151,69 +149,30 @@ def test_oracle_edge_cases():
     assert (fr.zbuf[fr.pix_to_face >= 0] - 2.0).abs().max() < 1e-6
 
 
-@pytest.mark.skipif(not have_reference(), reason='needs the reference checkout (/root/reference)')
 def test_restatements_match_reference_source():
-    """bit-for-bit against the reference's own code, read from the checkout at test time."""
-    nsb = extract('src/model/renderer.py', ['layered_rgb_blend'])
-    g = torch.Generator().manual_seed(9)
-    N, H, W, K = 2, 5, 7, 4
-    p2f = torch.randint(-1, 30, (N, H, W, K), generator=g)
-    d = torch.randn(N, H, W, K, generator=g) * 1e-4
-    col = torch.rand(N, H, W, K, 3, generator=g)
-    fa = torch.rand(40, generator=g)
-    for sigma in (0, 1e-4):
-        for ci in (True, False):
-            for a in (None, fa):
-                ref = nsb['layered_rgb_blend'](col, SimpleNamespace(pix_to_face=p2f, dists=d),
-                                               SimpleNamespace(sigma=sigma, background_color=(0.1, 0.2, 0.3)),
-                                               clip_inside=ci, faces_alpha=a)
-                assert torch.equal(ref, D.layered_rgb_blend(col, p2f, d, sigma, (0.1, 0.2, 0.3), ci, a))
-    ns = extract('src/utils/pytorch.py', ['signed_pow', 'safe_pow', 'SQRT_EPS'])
-    ns2 = extract('src/utils/superquadric.py', ['parametric_sq'], {'signed_pow': ns['signed_pow']})
-    eta, om = torch.rand(3, 42, generator=g) * 3 - 1.5, torch.rand(3, 42, generator=g) * 6 - 3
-    e1, e2 = torch.rand(3, 1, generator=g) * 1.8 + 0.1, torch.rand(3, 1, generator=g) * 1.8 + 0.1
-    assert torch.equal(ns2['parametric_sq'](eta, om, e1, e2), D.parametric_sq(eta, om, e1, e2))
-
-    class M:
-        def __init__(s, v, f): s.v, s.f = v, f
-        def get_mesh_verts_faces(s, i): return s.v, s.f
-    nsm = extract('src/utils/mesh.py', ['point_to_uv_sphericalmap', 'get_icosphere_uvs'],
-                  {'get_icosphere': lambda level: M(*pt3d.ico_sphere(level))})
+    """bit-for-bit against the outputs of the reference's own code (tests/golden/ref_restatements.npz)."""
+    from tests.golden.make_golden import BLEND_CASES
+    g = _npz('ref_restatements.npz')
+    col, p2f, d, fa = g['blend_colors'], g['blend_p2f'], g['blend_dists'], g['blend_faces_alpha']
+    for i, (sigma, ci, a) in enumerate(BLEND_CASES):
+        assert torch.equal(g[f'blend_out_{i}'], D.layered_rgb_blend(col, p2f, d, sigma, (0.1, 0.2, 0.3), ci, fa if a else None)), i
+    assert torch.equal(g['sq_out'], D.parametric_sq(g['sq_eta'], g['sq_omega'], g['sq_e1'], g['sq_e2']))
     for lvl in (1, 2):
-        f, uv = nsm['get_icosphere_uvs'](lvl, fix_continuity=True, fix_poles=True)
         fo, uvo = D.get_icosphere_uvs(lvl)
-        assert torch.equal(f, fo) and torch.equal(uv, uvo)
+        assert torch.equal(g[f'ico{lvl}_faces_uvs'], fo) and torch.equal(g[f'ico{lvl}_verts_uvs'], uvo)
 
 
-@pytest.mark.skipif(not have_reference(), reason='needs the reference checkout (/root/reference)')
 @pytest.mark.parametrize('coarse', [True, False])
 @pytest.mark.parametrize('tv_type', ['l2sq', 'l2', 'l1'])
 def test_regulariser_restatement_matches_reference_compute_losses(coarse, tv_type):
     """oracle.regularisers (parsimony / TV / overlap) against the reference's own DifferentiableBlocksWorld.compute_losses
-    (src/model/dbw.py:361-408), extracted with ast and run on a stand-in `self` that carries the state build_* leaves behind"""
-    ns = extract('src/utils/pytorch.py', ['safe_pow', 'SQRT_EPS'])
-    nsq = extract('src/utils/superquadric.py', ['implicit_sq'], {'safe_pow': ns['safe_pow']})
-    nsl = extract('src/model/loss.py', ['tv_norm_funcs'], {'safe_pow': ns['safe_pow']})
-    fn = extract_method('src/model/dbw.py', 'DifferentiableBlocksWorld', 'compute_losses',
-                        {'safe_pow': ns['safe_pow'], 'implicit_sq': nsq['implicit_sq'], 'OVERLAP_N_POINTS': 1000,
-                         'OVERLAP_N_BLOCKS': 1.95, 'OVERLAP_TEMPERATURE': 0.005})
+    (src/model/dbw.py:361-408) on the same parameters and overlap samples (tests/golden/ref_restatements.npz)"""
+    g = _npz('ref_restatements.npz')
     tpl = D.SceneTemplate(n_blocks=4, txt_size=16)
-    p = D.init_params(4, 16, seed=2, boxy=True)
-    p['alpha_logit'] = torch.tensor([3.0, 2.5, 2.0, -6.0])
-    p['T'] = p['T'] * 0.02                                           # crowd the blocks: the overlap term must be active
+    p = {k[len('reg_p_'):]: v for k, v in g.items() if k.startswith('reg_p_')}
     keep = torch.sigmoid(p['alpha_logit']) > 0.01                    # kill_blocks
-    alpha_full = torch.sigmoid(p['alpha_logit']) * keep
-    S, Rm = p['S'].exp() + tpl.scale_min, pt3d.rotation_6d_to_matrix(p['R_6d'])
-    eps = torch.sigmoid(p['sq_eps']) * 1.8 + 0.1
-    me = SimpleNamespace(loss_weights={'parsimony': 0.01, 'tv': 0.1, 'overlap': 1.0}, is_live=lambda name: coarse,
-                         _alpha_full=alpha_full, _bkg_maps=torch.sigmoid(p['texture_bkg']), _ground_maps=torch.sigmoid(p['texture_ground']),
-                         _blocks_maps=torch.sigmoid(p['textures']), tv_norm=nsl['tv_norm_funcs'][tv_type], n_blocks=4,
-                         ratio_block_scene=tpl.ratio, _blocks_SRT=(S, Rm, p['T']), _blocks_eps=(eps[:, :1], eps[:, 1:]))
-    torch.manual_seed(77)
-    ref = fn(me, torch.zeros(1, 3, 4, 4), torch.zeros(1, 3, 4, 4))
-    torch.manual_seed(77)
-    u01 = torch.rand(4, 1000, 3)
-    got = D.regularisers(tpl, p, coarse=coarse, keep=keep, tv_type=tv_type, unit_samples=u01, weights=(0.01, 0.1, 1.0))
+    ref = {k: g[f'reg_{int(coarse)}_{tv_type}_{k}'][0] for k in ('parsimony', 'tv', 'overlap')}
+    got = D.regularisers(tpl, p, coarse=coarse, keep=keep, tv_type=tv_type, unit_samples=g['reg_u01'], weights=(0.01, 0.1, 1.0))
     for k in ('parsimony', 'tv', 'overlap'):
         assert torch.allclose(got[k], ref[k], rtol=1e-6, atol=1e-9), (k, got[k].item(), ref[k].item())
     if coarse:

@@ -1,40 +1,11 @@
-"""CPU, authoring container only: the reference's UNMODIFIED trainer pipeline (src/trainer.py + optimizer.py + scheduler.py +
-utils/* + configs/dtu/scan24.yml) runs on this repo's model through the import shims of dbw_b200.compat.  See
-tests/ref_trainer_driver.py for what is swapped and why the render entry points are dummies when there is no GPU."""
-import json
+"""CPU: the import shims of dbw_b200.compat through which the reference's UNMODIFIED trainer pipeline (src/trainer.py +
+optimizer.py + scheduler.py + utils/*) runs on this repo's model.  tests/ref_trainer_driver.py runs that pipeline against
+a checkout of the reference."""
 import os
 import subprocess
 import sys
 
-import pytest
-
-from tests._refextract import have_reference
-
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-
-
-@pytest.mark.skipif(not have_reference(), reason='needs the reference checkout (/root/reference)')
-def test_unmodified_reference_trainer_runs_on_the_drop_in_model(tmp_path):
-    run_dir = tmp_path / 'runs' / 'synthetic' / 'b200'
-    run_dir.parent.mkdir(parents=True)
-    res = subprocess.run([sys.executable, os.path.join(ROOT, 'tests', 'ref_trainer_driver.py'), str(run_dir), '--iters', '3'],
-                         capture_output=True, text=True, timeout=600)
-    assert res.returncode == 0, res.stdout[-3000:] + res.stderr[-3000:]
-    line = [l for l in res.stdout.splitlines() if l.startswith('DRIVER_RESULT ')][-1]
-    out = json.loads(line[len('DRIVER_RESULT '):])
-    # the loss columns of configs/dtu/scan24.yml, in the reference's order (dbw.py:145-157)
-    assert out['loss_names'] == ['loss_rgb', 'loss_perceptual', 'loss_parsimony', 'loss_tv', 'loss_overlap', 'loss_total']
-    # optimizer.py:9-14: the `texture*` parameters form the second Adam group with their own learning rate
-    assert out['param_groups'] == [7, 3] and out['lrs'] == [5e-3, 5e-2]
-    assert {'textures', 'texture_bkg', 'texture_ground', 'S', 'T', 'R_6d', 'alpha_logit'} <= set(out['moved'])
-    assert out['cur_epoch'] == 1 and out['model_name'] == 'dbw'
-    # checkpoint keys = the reference's parameter / buffer names (SURVEY 8b)
-    assert {'sq_eps', 'R_6d_ground', 'T_ground', 'S', 'R_6d', 'T', 'alpha_logit', 'texture_bkg', 'texture_ground', 'textures',
-            'R_world', 'T_world', 'bkg_verts_uvs', 'ground_verts_uvs', 'sq_eta', 'sq_omega', 'block_faces_uvs',
-            'block_verts_uvs'} <= set(out['checkpoint_keys'])
-    assert out['train_metrics_rows'] >= 3 and out['val_metrics_rows'] == 2
-    assert out['resumed_epoch_start'] == 2 and out['resume_equal']
-    assert 'pytorch3d' in out['shimmed'] and 'toolz' in out['shimmed']
 
 
 def test_compat_shims_are_thin_and_fail_loudly():
